@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — frame-pairs/s of the per-video test-time optimisation step (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--pairs B] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--pairs B] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = one joint-phase optimisation step (depth net + scene-flow MLP trainable, flags of
 experiments/davis/train_sequence.sh) over B synthetic frame pairs per GPU (default 384x224, 80 frames =
@@ -66,7 +66,14 @@ def parse():
     ap.add_argument('--no-extras', action='store_true', help='skip the B=1 line, the eager-GPU reference and the kernel rooflines')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--roofline-pairs', type=int, default=64)
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)')
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs needs --impl b200')
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -276,6 +283,40 @@ def gpu_eager_reference(dev, B, n_steps=8, warmup=3):
 
 
 # ---------------------------------------------------------------------------------------------------
+DUMP_LOSSES = ('loss', 'flow_loss_1_2', 'disp_loss_1_2', 'sf_loss', 'acc_reg')
+DUMP_DEPTH_SAMPLE = 1 << 20    # depth-net values kept per array (of ~105 M); the MLP's ~0.3 M are kept whole
+
+
+def dump_outputs(out_dir, log, model):
+    """What the last timed step hands its caller, as out_dir/<name>.npy: its loss terms (float64 scalars, the batch log), and
+    the model state it leaves behind, which is what a checkpoint of the run would hold - parameters and both Adam moments of
+    the scene-flow MLP in full, and of the depth net a fixed sample (the same DUMP_DEPTH_SAMPLE positions, drawn with seed 0,
+    for every array and run), float32, in state-dict order. With the same arguments the inputs are identical from run to run,
+    so two builds can be compared array by array."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for k in DUMP_LOSSES:
+        np.save(os.path.join(out_dir, k + '.npy'), np.float64(log[k]))
+    for tag, net, opt_ in (('depth_net', model.net_depth, model.optimizer_depth),
+                           ('sceneflow_mlp', model.net_sceneflow, model.optimizer_scene)):
+        params = [p for _, p in net.named_parameters()]
+        st = opt_.state_dict()['state']
+        moments = {key: [st[i][key] if i in st else torch.zeros_like(p) for i, p in enumerate(params)]
+                   for key in ('exp_avg', 'exp_avg_sq')}
+        arrays = {'params': params, 'adam_exp_avg': moments['exp_avg'], 'adam_exp_avg_sq': moments['exp_avg_sq']}
+        n = sum(p.numel() for p in params)
+        idx = None
+        if n > DUMP_DEPTH_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(n, DUMP_DEPTH_SAMPLE, replace=False))
+            idx = torch.from_numpy(idx).to(params[0].device)
+        for name, ts in arrays.items():
+            v = torch.cat([t.detach().reshape(-1).float() for t in ts])
+            if idx is not None:
+                v = v[idx]
+            np.save(os.path.join(out_dir, '%s_%s.npy' % (tag, name)), v.cpu().numpy())
+
+
 def roofline_reproject(pairs, hbm_peak, peak_kind):
     """Fused re-projection kernels on a batch >> L2 (pairs x 344 KB x 8 tensors), L2 flushed between launches,
     CUDA events on the launching (current) stream."""
@@ -502,6 +543,8 @@ def run_b200_arm(args):
     host, resident = make_batches(B, Wm + K)
     # (1) device-resident inputs: the headline `value`
     t_dev, logs, clocks, launches = timed(resident, Wm, K, ClockSampler(local))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, logs[-1], model)
     # (2) end to end through the plug-in call with HOST (pinned) batches: H2D + D2H inside the timed region
     t_e2e, logs2, _, _ = timed(host, Wm, K)
     h2d = sum(v.numel() * v.element_size() for v in host[Wm].values() if torch.is_tensor(v))
@@ -509,12 +552,11 @@ def run_b200_arm(args):
     # (3) the reference's own schedule: ONE pair per step (train_sequence.sh:29-34), same gap cycle
     b1 = None
     if not args.no_extras and B != 1:
-        K1 = max(K, 10)
-        host1, res1 = make_batches(1, Wm + K1)
-        t1_dev, _, _, l1 = timed(res1, Wm, K1)
-        t1_e2e, _, _, _ = timed(host1, Wm, K1)
-        b1 = {'value': K1 * world / t1_dev, 'unit': UNIT, 'ms_per_step': 1e3 * t1_dev / K1, 'steps': K1,
-              'e2e': K1 * world / t1_e2e, 'gpu_launches_per_step': l1 / K1,
+        host1, res1 = make_batches(1, Wm + K)
+        t1_dev, _, _, l1 = timed(res1, Wm, K)
+        t1_e2e, _, _, _ = timed(host1, Wm, K)
+        b1 = {'value': K * world / t1_dev, 'unit': UNIT, 'ms_per_step': 1e3 * t1_dev / K, 'steps': K,
+              'e2e': K * world / t1_e2e, 'gpu_launches_per_step': l1 / K,
               'what': 'this arm at 1 pair per step per GPU (the batch the reference DataLoader delivers), same gap cycle'}
         del host1, res1
     if rank != 0:
@@ -533,7 +575,7 @@ def run_b200_arm(args):
         del host, resident
         torch.cuda.empty_cache()
         if world == 1:
-            gref = gpu_eager_reference(dev, B)
+            gref = gpu_eager_reference(dev, B, n_steps=K)
             if 'pairs_per_step_%d' % B in gref:
                 gref['speedup_value_vs_eager_same_batch'] = value / gref['pairs_per_step_%d' % B]
                 gref['speedup_value_vs_eager_1_pair_per_step'] = value / gref['pairs_per_step_1']

@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE — generates tests/golden/*.pt by executing the UNMODIFIED reference
 (/root/reference, imported through oracle/ref_harness.py) on seeded synthetic inputs.
 
-Run in the authoring container only:   python -m oracle.gen_golden [reproject|mlp|step|all]
+Run where the reference tree is available:   python -m oracle.gen_golden [reproject|mlp|modules|step|all]
 The fixtures are small (tens of KB .. a few MB) and committed; the GPU box never sees /root/reference.
 Tensors are stored channel-planar ([B,C,H,W]) to match the C ABI layout.
 """
@@ -189,6 +189,114 @@ def gen_mlp():
     print('wrote mlp_golden.pt acc_reg=%g |sf|max=%g' % (val, out['multi_3']['sf'].abs().max()))
 
 
+def geometry_inputs(dtype):
+    """Inputs of the module-level geometry comparison (tests/test_oracle_vs_reference.py), all from seeds; the float32 set is
+    the float64 set rounded."""
+    from dvd_b200 import synthetic
+    B, H, W = 2, 40, 56
+    b = synthetic.make_batch([(3, 5), (10, 18)], H=H, W=W, dtype=dtype, leading_dim=False, flow_sigma=6.0)
+    d1 = synthetic.make_depths(B, H, W, seed=1, dtype=dtype)
+    d2 = synthetic.make_depths(B, H, W, seed=2, dtype=dtype)
+    d1[0, 0, :3, :5] = 150.0
+    d1[1, 0, 10:12, :] = -1.0
+    sf = (torch.randn(B, 3, H, W, generator=torch.Generator().manual_seed(3), dtype=torch.float64) * 0.05).to(dtype)
+    return b, d1, d2, sf
+
+
+def depth_net_input():
+    return torch.rand(2, 3, 64, 96, generator=torch.Generator().manual_seed(4))
+
+
+def mlp_inputs_small():
+    g = torch.Generator().manual_seed(5)
+    return torch.randn(1, 3, 9, 11, generator=g) * 3, torch.full((1, 1, 9, 11), 0.4)
+
+
+# checkpoint skeleton: tensors above this size are stored as (shape, dtype) and refilled from a seed by the test
+SKELETON_MAX_NUMEL = 16
+
+
+def checkpoint_skeleton(obj):
+    """Everything of a checkpoint except the values of its large tensors: containers, keys, order, small tensors verbatim."""
+    if torch.is_tensor(obj):
+        if obj.numel() > SKELETON_MAX_NUMEL:
+            return ('seeded_tensor', tuple(obj.shape), str(obj.dtype).replace('torch.', ''))
+        return obj.clone()
+    if isinstance(obj, dict):
+        return {k: checkpoint_skeleton(v) for k, v in obj.items()}
+    if isinstance(obj, (list, tuple)):
+        return type(obj)(checkpoint_skeleton(v) for v in obj)
+    return obj
+
+
+def checkpoint_from_skeleton(obj, g):
+    """Inverse of checkpoint_skeleton: large tensors refilled, in traversal order, from generator `g` (second moments >= 0)."""
+    if isinstance(obj, tuple) and len(obj) == 3 and obj[0] == 'seeded_tensor':
+        t = torch.randn(obj[1], generator=g, dtype=torch.float64)
+        return t.to(getattr(torch, obj[2]))
+    if isinstance(obj, dict):
+        return {k: (checkpoint_from_skeleton(v, g).abs() if k == 'exp_avg_sq' else checkpoint_from_skeleton(v, g))
+                for k, v in obj.items()}
+    if isinstance(obj, (list, tuple)):
+        return type(obj)(checkpoint_from_skeleton(v, g) for v in obj)
+    return obj
+
+
+def gen_reference_modules():
+    """Outputs of the reference's own modules that tests/test_oracle_vs_reference.py compares the oracle and the mirrors with."""
+    import tempfile
+    from dvd_b200 import synthetic
+    ns = ref_harness.import_reference()
+    # geometry modules: flow_by_depth + scene_flow_projection_slack, float32 and float64
+    for dtype in (torch.float32, torch.float64):
+        b, d1, d2, sf = geometry_inputs(dtype)
+        H, W = d1.shape[-2:]
+        fb, sl = ns.sfp.flow_by_depth(), ns.sfp.scene_flow_projection_slack()
+        if dtype == torch.float64:
+            yy, xx = torch.meshgrid(torch.arange(H).double(), torch.arange(W).double(), indexing='ij')
+            coord = torch.ones([1, H, W, 1, 3], dtype=dtype)
+            coord[0, ..., 0, 0], coord[0, ..., 0, 1] = xx, yy
+            fb.coord, sl.coord = coord, coord.clone()
+        pose = {k: b[k] for k in ('R_1', 'R_2', 'R_1_T', 'R_2_T', 't_1', 't_2', 'K', 'K_inv')}
+        r1 = fb(depth_1=d1, depth_2=d2, flow_1_2=b['flow_1_2'], **pose)
+        sfl = sf.permute(0, 2, 3, 1)[..., None, :]
+        r2 = sl(depth_1=d1, depth_2=d2, flow_1_2=b['flow_1_2'], flow_2_1=b['flow_2_1'], sflow_1_2=sfl, sflow_2_1=sfl, **pose)
+        ref = {'global_p1': _cf(r1['global_p1']), 'sf_by_depth': _cf(r1['sf_by_depth']),
+               'warped_p2_camera_2': _cf(r2['warped_p2_camera_2']), 'p1_camera_2': _cf(r2['p1_camera_2']),
+               'dflow_1_2': r2['dflow_1_2'].permute(0, 3, 1, 2).contiguous(),
+               'staticflow_1_2': r2['staticflow_1_2'].permute(0, 3, 1, 2).contiguous(),
+               'depth_image_1_2': r2['depth_image_1_2'].contiguous(), 'depth_warp_1_2': r2['depth_warp_1_2'].contiguous()}
+        name = 'ref_geometry_%s.pt' % str(dtype).replace('torch.', '')
+        torch.save({k: v.detach().clone() for k, v in ref.items()}, os.path.join(GOLD, name))
+        print('wrote', name)
+    out = {}
+    # depth nets with name-seeded weights: parameter names / shapes and outputs
+    x = depth_net_input()
+    midas = synthetic.seed_net_(ns.midas.MidasNet(path=None, non_negative=True, normalize_input=True), 0, 2000.0).eval()
+    hg = synthetic.seed_net_(ns.hourglass.HourglassModel_Embed(noexp=False), 0)
+    hg.defrost()
+    with torch.no_grad():
+        out['midas'] = {'keys': [(k, tuple(v.shape)) for k, v in midas.state_dict().items()], 'out': midas(x.clone())}
+        out['hourglass'] = {'keys': [(k, tuple(v.shape)) for k, v in hg.state_dict().items()], 'out': hg(x.clone())}
+    # scene-flow MLP with name-seeded weights
+    net = synthetic.seed_net_(ns.sff.SceneFlowFieldNet(net_width=256, n_layers=4, time_dependent=True, N_freq_xyz=16,
+                                                       N_freq_t=16), 3)
+    p, t = mlp_inputs_small()
+    with torch.no_grad():
+        out['mlp'] = {'keys': [(k, tuple(v.shape)) for k, v in net.state_dict().items()], 'out': net(p, t)}
+    # a checkpoint written by the reference's NetInterface.save_state_dict after one optimisation step (hourglass variant)
+    opt = ref_harness.default_opt(midas=False, lr=1e-4)
+    ref_model, _ = ref_harness.build_reference_model(opt, seed=0)
+    batch = synthetic.make_batch([(3, 5)], H=32, W=48, seed=1, smooth_flow=True)
+    ref_model._train_on_batch(6, 0, {k: (v.clone() if torch.is_tensor(v) else v) for k, v in batch.items()})
+    with tempfile.TemporaryDirectory() as d:
+        f = os.path.join(d, 'ref.pt')
+        ref_model.save_state_dict(f, save_optimizer=True, additional_values={'epoch': 6})
+        out['checkpoint'] = checkpoint_skeleton(torch.load(f, map_location='cpu', weights_only=False))
+    torch.save(out, os.path.join(GOLD, 'ref_modules.pt'))
+    print('wrote ref_modules.pt')
+
+
 if __name__ == '__main__':
     what = sys.argv[1] if len(sys.argv) > 1 else 'all'
     os.makedirs(GOLD, exist_ok=True)
@@ -196,6 +304,8 @@ if __name__ == '__main__':
         gen_reproject()
     if what in ('mlp', 'all'):
         gen_mlp()
+    if what in ('modules', 'all'):
+        gen_reference_modules()
     if what in ('step', 'all'):
         from oracle import gen_golden_step
         gen_golden_step.main()

@@ -1,9 +1,9 @@
 """Checkpoint hand-over with the reference (models/netinterface.py:528-574): a file in the reference's layout - net state dicts
 under the reference's parameter names plus `torch.optim.Adam.state_dict()`s, exactly what `NetInterface.save_state_dict` writes -
 is loaded into the dvd_b200 Model; the next Adam step on the flat buffers then equals torch.optim.Adam's on the same gradient, and
-the state written back is loadable by torch.optim.Adam again. (The file is produced here with torch itself because the reference
-tree does not exist on the GPU box; tests/test_oracle_vs_reference.py::test_reference_written_checkpoint_loads does the same with
-a file written by the reference's own NetInterface when /root/reference is present.)"""
+the state written back is loadable by torch.optim.Adam again. (The file is produced here with torch itself;
+tests/test_oracle_vs_reference.py::test_reference_written_checkpoint_loads does the same with the layout of a file written by the
+reference's own NetInterface.)"""
 import pytest
 import torch
 

@@ -1,108 +1,87 @@
-"""CPU, authoring container only (skipped where /root/reference is absent, e.g. on the GPU box): the oracle
-restatement and the host-side mirrors against the UNMODIFIED reference code imported through
-oracle/ref_harness.py. The same comparisons, frozen, are the committed fixtures in tests/golden/."""
+"""CPU: the oracle restatement and the host-side mirrors against outputs of the UNMODIFIED reference code, stored in
+tests/golden/ref_*.pt by oracle/gen_golden.py (`python -m oracle.gen_golden modules`, which imports the reference through
+oracle/ref_harness.py). Inputs and name-seeded weights are rebuilt here from the same seeds."""
+import os
+
 import pytest
 import torch
 
-from conftest import rel_err
-from oracle import ref_harness
+from conftest import GOLDEN, rel_err
+from oracle import gen_golden
 
-pytestmark = pytest.mark.skipif(not ref_harness.reference_available(), reason='reference tree not present')
+
+def _load(name):
+    return torch.load(os.path.join(GOLDEN, name), weights_only=False)
 
 
 @pytest.fixture(scope='module')
-def ns():
-    return ref_harness.import_reference()
+def ref_modules():
+    return _load('ref_modules.pt')
 
 
-def _cf(x):
-    return x.squeeze(3).permute(0, 3, 1, 2)
+def _keys(sd):
+    return [(k, tuple(v.shape)) for k, v in sd.items()]
 
 
 @pytest.mark.parametrize('dtype', [torch.float32, torch.float64])
-def test_geometry_matches_reference_modules(ns, dtype):
-    from dvd_b200 import synthetic
+def test_geometry_matches_reference_modules(dtype):
     from oracle import geometry
-    B, H, W = 2, 40, 56
-    b = synthetic.make_batch([(3, 5), (10, 18)], H=H, W=W, dtype=dtype, leading_dim=False, flow_sigma=6.0)
-    d1 = synthetic.make_depths(B, H, W, seed=1, dtype=dtype)
-    d2 = synthetic.make_depths(B, H, W, seed=2, dtype=dtype)
-    d1[0, 0, :3, :5] = 150.0
-    d1[1, 0, 10:12, :] = -1.0
-    sf = torch.randn(B, 3, H, W, dtype=dtype) * 0.05
-    fb, sl = ns.sfp.flow_by_depth(), ns.sfp.scene_flow_projection_slack()
-    if dtype == torch.float64:
-        yy, xx = torch.meshgrid(torch.arange(H).double(), torch.arange(W).double(), indexing='ij')
-        coord = torch.ones([1, H, W, 1, 3], dtype=dtype)
-        coord[0, ..., 0, 0], coord[0, ..., 0, 1] = xx, yy
-        fb.coord, sl.coord = coord, coord.clone()
-    pose = {k: b[k] for k in ('R_1', 'R_2', 'R_1_T', 'R_2_T', 't_1', 't_2', 'K', 'K_inv')}
-    r1 = fb(depth_1=d1, depth_2=d2, flow_1_2=b['flow_1_2'], **pose)
-    sfl = sf.permute(0, 2, 3, 1)[..., None, :]
-    r2 = sl(depth_1=d1, depth_2=d2, flow_1_2=b['flow_1_2'], flow_2_1=b['flow_2_1'], sflow_1_2=sfl, sflow_2_1=sfl, **pose)
+    b, d1, d2, sf = gen_golden.geometry_inputs(dtype)
+    ref = _load('ref_geometry_%s.pt' % str(dtype).replace('torch.', ''))
     o = geometry.reproject(d1, d2, sf, b)
     tol = 5e-6 if dtype == torch.float32 else 1e-12
-    ref = {'global_p1': _cf(r1['global_p1']), 'sf_by_depth': _cf(r1['sf_by_depth']),
-           'warped_p2_camera_2': _cf(r2['warped_p2_camera_2']), 'p1_camera_2': _cf(r2['p1_camera_2']),
-           'dflow_1_2': r2['dflow_1_2'].permute(0, 3, 1, 2), 'staticflow_1_2': r2['staticflow_1_2'].permute(0, 3, 1, 2),
-           'depth_image_1_2': r2['depth_image_1_2'], 'depth_warp_1_2': r2['depth_warp_1_2']}
     for k, v in ref.items():
+        assert v.dtype == dtype
         assert rel_err(o[k], v) < tol, k
 
 
-def test_depth_net_mirrors_and_functional_oracle_match_reference(ns):
+def test_depth_net_mirrors_and_functional_oracle_match_reference(ref_modules):
     from dvd_b200 import synthetic
     from dvd_b200.third_party import MiDaS as M, hourglass as HG
     from oracle import depth_nets
-    x = torch.rand(2, 3, 64, 96)
-    ref = synthetic.seed_net_(ns.midas.MidasNet(path=None, non_negative=True, normalize_input=True), 0, 2000.0).eval()
+    x = gen_golden.depth_net_input()
+    # name-seeded weights: the same parameter names and shapes as the reference's nets mean the same values
     mine = synthetic.seed_net_(M.MidasNet(non_negative=True, normalize_input=True), 0, 2000.0).eval()
-    assert list(ref.state_dict()) == list(mine.state_dict())
+    assert _keys(mine.state_dict()) == ref_modules['midas']['keys']
+    a = ref_modules['midas']['out']
     with torch.no_grad():
-        a = ref(x.clone())
         # the MiDaS mirror only holds parameters (all of its arithmetic is CUDA: depth_engine.py); on the CPU its state dict
         # drives the functional oracle, and it refuses to run itself
         assert rel_err(depth_nets.midas_forward(mine.state_dict(), x), a) < 1e-5
-        assert rel_err(depth_nets.midas_forward(ref.state_dict(), x), a) < 1e-5
-        import pytest
         with pytest.raises(RuntimeError):
             mine(x)
-    rh = synthetic.seed_net_(ns.hourglass.HourglassModel_Embed(noexp=False), 0)
     mh = synthetic.seed_net_(HG.HourglassModel_Embed(noexp=False), 0)
-    assert list(rh.state_dict()) == list(mh.state_dict())
-    rh.defrost(), mh.defrost()
+    assert _keys(mh.state_dict()) == ref_modules['hourglass']['keys']
+    mh.defrost()
+    a = ref_modules['hourglass']['out']
     with torch.no_grad():
-        a = rh(x.clone())
         assert rel_err(mh(x), a) < 1e-6
-        assert rel_err(depth_nets.hourglass_forward(rh.state_dict(), x), a) < 1e-5
+        assert rel_err(depth_nets.hourglass_forward(mh.state_dict(), x), a) < 1e-5
 
 
-def test_mlp_oracle_matches_reference_module(ns):
+def test_mlp_oracle_matches_reference_module(ref_modules):
+    from dvd_b200 import synthetic
+    from dvd_b200.networks.sceneflow_field import SceneFlowFieldNet
     from oracle import sf_mlp
-    torch.manual_seed(3)
-    net = ns.sff.SceneFlowFieldNet(net_width=256, n_layers=4, time_dependent=True, N_freq_xyz=16, N_freq_t=16)
-    p = torch.randn(1, 3, 9, 11) * 3
-    t = torch.full((1, 1, 9, 11), 0.4)
+    net = synthetic.seed_net_(SceneFlowFieldNet(net_width=256, n_layers=4, time_dependent=True, N_freq_xyz=16, N_freq_t=16), 3)
+    assert _keys(net.state_dict()) == ref_modules['mlp']['keys']
+    p, t = gen_golden.mlp_inputs_small()
     with torch.no_grad():
-        assert rel_err(sf_mlp.mlp_forward(p, t, sf_mlp.layers_from_state_dict(net.state_dict())), net(p, t)) < 1e-5
+        assert rel_err(sf_mlp.mlp_forward(p, t, sf_mlp.layers_from_state_dict(net.state_dict())), ref_modules['mlp']['out']) < 1e-5
 
 
-def test_reference_written_checkpoint_loads(tmp_path):
-    """A checkpoint written by the REFERENCE's own `NetInterface.save_state_dict` (models/netinterface.py:528-536) after one of its
-    optimisation steps loads into the dvd_b200 Model: same net keys / values, and its two torch.optim.Adam state dicts map onto the
-    flat Adam buffers (exp_avg, exp_avg_sq, step) and come back out identical. Hourglass variant (21 MB instead of 420 MB)."""
+def test_reference_written_checkpoint_loads(ref_modules, tmp_path):
+    """A checkpoint in the layout the REFERENCE's own `NetInterface.save_state_dict` (models/netinterface.py:528-536) wrote after
+    one of its optimisation steps loads into the dvd_b200 Model: same net keys / values, and its two torch.optim.Adam state dicts
+    map onto the flat Adam buffers (exp_avg, exp_avg_sq, step) and come back out identical. Hourglass variant. The fixture keeps
+    the file's whole structure (containers, keys, order, which parameters have optimiser state, small tensors); the values of
+    the large tensors are refilled from a seed."""
     from dvd_b200 import synthetic
     from dvd_b200.flat import FlatAdam, FlatParams
     from dvd_b200.models import get_model
-    opt = ref_harness.default_opt(midas=False, lr=1e-4)
-    ref_model, _ = ref_harness.build_reference_model(opt, seed=0)
-    batch = synthetic.make_batch([(3, 5)], H=32, W=48, seed=1, smooth_flow=True)
-    ref_model._train_on_batch(6, 0, {k: (v.clone() if torch.is_tensor(v) else v) for k, v in batch.items()})
+    ref_sd = gen_golden.checkpoint_from_skeleton(ref_modules['checkpoint'], torch.Generator().manual_seed(0))
     f = str(tmp_path / 'ref.pt')
-    ref_model.save_state_dict(f, save_optimizer=True, additional_values={'epoch': 6})
-    ref_sd = torch.load(f, map_location='cpu', weights_only=False)
-    import dvd_b200.models.scene_flow_motion_field as mine_mod
-    mine_mod.depth_pretrain_path = None       # (with the reference on sys.path its configs/__init__.py names a file that is not here)
+    torch.save(ref_sd, f)
     mine = get_model('scene_flow_motion_field')(synthetic.default_opt(midas=False, lr=1e-4), None)
     extra = mine.load_state_dict(f)
     assert extra.get('epoch') == 6
